@@ -7,6 +7,7 @@
              through all S iterations (gibbs -> H -> L leapfrog steps -> H -> MH -> sample write), = C*S*L chain-steps
 
     python bench.py --gpus N --steps K --warmup W            (under torchrun for N > 1: one rank per GPU)
+    python bench.py ... --dump-outputs DIR                    (+ the last timed step's outputs as DIR/<name>.npy)
     python bench.py --impl reference ...                      (the reference's algorithm on the host cores)
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
@@ -531,6 +532,23 @@ def other_configs(dev, rank, world):
 # ----------------------------------------------------------------------------------------------------------
 # B200 arm
 # ----------------------------------------------------------------------------------------------------------
+DUMP_SLOT_STRIDE = 32
+
+
+def dump_outputs(dirname, res):
+    """--dump-outputs: what engine.hmc_run returned for the last timed step (rank 0's chains), one float32 .npy per
+    array.  Of the (C, S, D) sample block (1 GiB) every chain's slots 0, 32, 64, ... and the last slot are written
+    (33 of S = 1000, 33 MiB); the other arrays are written whole: final_state (C, D), accepted and diverged (C, S),
+    step_size and num_rejected (C,).  The inputs depend only on the seeds in this file and --steps, so two builds run
+    with the same arguments can be compared file by file."""
+    import numpy as np
+    slots = sorted(set(range(0, S, DUMP_SLOT_STRIDE)) | {S - 1})
+    arrays = {'samples': res.samples[:, slots], 'final_state': res.final_state, 'accepted': res.accepted,
+              'diverged': res.diverged, 'step_size': res.step_size, 'num_rejected': res.num_rejected}
+    for name, t in arrays.items():
+        np.save(os.path.join(dirname, name + '.npy'), t.float().cpu().numpy())
+
+
 def run_b200_arm(args, rank, world, local_rank):
     import torch.distributed as dist
     import hamiltorch_b200 as hb
@@ -654,10 +672,14 @@ def run_b200_arm(args, rank, world, local_rank):
         # drop the result before the next call allocates its (small) output tensors: with two result sets alive the
         # caching allocator has to cudaMalloc a new segment inside the timed region, and cudaMalloc behind a full launch
         # queue was measured at 7 - 436 ms (always in the second timed step) against 1.51 ms for every other step
-        res = None
+        if k + 1 < args.steps:
+            res = None
     gather_stats()
     ev[-1].record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res)         # before the legs below overwrite `out`, which holds res.samples
+    res = None
     t_total_ms = ev[0].elapsed_time(ev[-1])
     step_ms = [ev[1 + 2 * k].elapsed_time(ev[2 + 2 * k]) for k in range(args.steps)]
     t_kernel_ms = sum(step_ms) / args.steps
@@ -914,7 +936,15 @@ def main():
                     help='N > 1: skip the timed all-gather of every step\'s samples (value_with_gather)')
     ap.add_argument('--no-other-configs', action='store_true', help='skip BASELINE configs 3 / 4 / 5')
     ap.add_argument('--no-numa-bind', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='B200 arm: write the outputs of the last timed step to DIR/<name>.npy (see dump_outputs)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs:
+        if args.impl != 'b200':
+            ap.error('--dump-outputs applies to the B200 arm')
+        os.makedirs(args.dump_outputs, exist_ok=True)      # fail before any GPU work if DIR cannot be created
     rank = int(os.environ.get('RANK', '0'))
     world = int(os.environ.get('WORLD_SIZE', '1'))
     local_rank = int(os.environ.get('LOCAL_RANK', '0'))

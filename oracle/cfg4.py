@@ -5,8 +5,8 @@ eps=5e-4, L=10, inv_mass=ones(D), tau_out=100, tau_list=[1,1,1,1].
 The fixture would be 27 MB per 8 x 100 chain block, so the GPU tests run this oracle LIVE on the GPU box's host cores
 (one process per chain); the random stream of a chain is a seeded CPU torch.Generator, identical on every machine with
 this torch build.  sample_hmc's split branch is pinned bit-identical to the unmodified reference by
-oracle/gen_golden.py (tests/golden/mlp_split_*.npz) and, at this exact configuration, by
-tests/test_oracle_golden.py::test_cfg4_oracle_equals_reference_live in the build container."""
+oracle/gen_golden.py (tests/golden/mlp_split_*.npz) and, at this exact configuration, by oracle/ref_pins.py
+(tests/test_oracle_golden.py::test_cfg4_oracle_equals_reference_live)."""
 import torch
 
 M, L, EPS, TAU_OUT, N_ROWS, N_IN, HID = 4, 10, 5e-4, 100., 1024, 64, 128

@@ -1,9 +1,8 @@
 """ORACLE -- TEST INFRASTRUCTURE ONLY.
 
-Imports the UNMODIFIED reference (AdamCobb/hamiltorch @ 19b627b) from /root/reference.  That tree only exists
-in the build container, never on the GPU box: nothing under tests/ -m gpu, smoke() or bench.py may call this.
-It is used by oracle/gen_golden.py (fixture generation) and by CPU tests that are skipped when the tree is
-absent.
+Imports the UNMODIFIED reference (AdamCobb/hamiltorch @ 19b627b) from REFERENCE_ROOT.  Only the fixture generators
+(oracle/gen_golden.py, oracle/gen_cfg3.py, oracle/ref_pins.py) call this; the tests, smoke() and bench.py compare
+against what they stored under tests/golden/ and never need the reference tree.
 
 The reference needs ``termcolor`` (util.py:4, used only by eval_print) which is not installed here; a two-line
 shim module is injected into sys.modules (SURVEY.md section 8c).  torch.distributions argument validation is

@@ -58,6 +58,33 @@ def test_reference_arm_is_bounded_and_survives_sigterm():
     assert d['impl'] == 'reference' and d['cut_short'] is True and d['steps_completed'] < 400
 
 
+def test_dump_outputs_writes_what_the_timed_call_returned(tmp_path):
+    """--dump-outputs: float32 .npy files of an engine.hmc_run result, the sample block reduced to every chain's slots
+    0, 32, 64, ... and the last slot (here a CPU stand-in of config 2's shapes with 3 chains)."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    from hamiltorch_b200.engine import HMCResult
+    C, S, D, ld = 3, bench.S, 6, 8
+    g = torch.Generator().manual_seed(0)
+    res = HMCResult(torch.randn(C, S, ld, generator=g), (torch.rand(C, S, generator=g) < 0.9).to(torch.uint8),
+                    torch.zeros(C, S, dtype=torch.uint8), None, torch.full((C,), 0.05),
+                    torch.tensor([3, 0, 7], dtype=torch.int32), D, S)
+    res.final_state = torch.randn(C, ld, generator=g)[:, :D]
+    bench.dump_outputs(str(tmp_path), res)
+    got = {f[:-4]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert set(got) == {'samples', 'final_state', 'accepted', 'diverged', 'step_size', 'num_rejected'}
+    assert all(a.dtype == np.float32 for a in got.values())
+    slots = list(range(0, S, 32)) + [S - 1]
+    assert np.array_equal(got['samples'], res.samples[:, slots].numpy())
+    assert np.array_equal(got['final_state'], res.final_state.numpy())
+    assert np.array_equal(got['accepted'], res.accepted.float().numpy())
+    assert got['num_rejected'].tolist() == [3, 0, 7]
+    # at config 2's size (256 chains, D = 1024) all files together stay within 64 MiB
+    assert 4 * bench.C_PER_GPU * (len(slots) * bench.D + bench.D + 2 * S + 2) <= 64 << 20
+
+
 def test_host_topology_helpers():
     sys.path.insert(0, ROOT)
     import bench

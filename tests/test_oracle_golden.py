@@ -1,13 +1,12 @@
 """CPU: pin the oracle (oracle/hmc_oracle.py) against fixtures produced by the UNMODIFIED reference
-(oracle/gen_golden.py), and -- when /root/reference is present -- against the reference itself, live."""
+(oracle/gen_golden.py), and against the reference's own output under the same torch RNG state (oracle/ref_pins.py)."""
 import os
 
 import numpy as np
 import pytest
 import torch
 
-from oracle import cases, hmc_oracle as O
-from oracle.ref_import import reference_available, import_reference
+from oracle import cases, hmc_oracle as O, ref_pins
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 
@@ -77,24 +76,20 @@ def test_dual_average_first_steps():
     assert abs(H2 - ((1 - 1 / 12) * H + (1 / 12) * 0.8)) < 1e-15
 
 
-@pytest.mark.skipif(not reference_available(), reason='/root/reference only exists in the build container')
 def test_oracle_equals_reference_live():
-    """Bit-for-bit: oracle.sample_hmc == hamiltorch.sample under the same torch RNG state (HMC and HMC_NUTS)."""
+    """Bit-for-bit: oracle.sample_hmc == hamiltorch.sample under the same torch RNG state (HMC and HMC_NUTS), against
+    the reference's output stored by oracle/ref_pins.py."""
     torch.set_num_threads(1)
-    ref = import_reference()
-    from hamiltorch_b200 import targets as T
-    tgt = T.GaussianDiag(torch.linspace(-1, 1, 12), 0.3 + torch.rand(12, generator=torch.Generator().manual_seed(0)))
-    init = torch.zeros(12)
+    d = np.load(ref_pins.PINS)
     for nuts in (False, True):
-        kw = dict(num_samples=25, num_steps_per_sample=4, step_size=0.4, burn=8)
-        torch.manual_seed(99)
-        r = ref.sample(log_prob_func=tgt, params_init=init, verbose=False, debug=2,
-                       sampler=ref.Sampler.HMC_NUTS if nuts else ref.Sampler.HMC, **kw)
-        torch.manual_seed(99)
-        o = O.sample_hmc(tgt, init, nuts=nuts, **kw)
-        assert torch.equal(torch.stack(r[0]), torch.stack(o['samples']))
+        tag = 'nuts' if nuts else 'hmc'
+        o = ref_pins.oracle_gauss12(nuts)
+        assert torch.equal(torch.from_numpy(d['gauss12_%s_samples' % tag]), torch.stack(o['samples']))
         if nuts:
-            assert r[1] == o['step_size']
+            assert float(d['gauss12_nuts_extra']) == o['step_size']
+        else:                                # the reference's acceptance rate
+            rate = 1 - o['num_rejected'] / ref_pins.GAUSS12_KW['num_samples']
+            assert abs(float(d['gauss12_hmc_extra']) - rate) < 1e-12
 
 
 # ---- sampler=RMHMC: oracle/rmhmc_oracle.py ---------------------------------------------------------------------
@@ -146,23 +141,9 @@ def test_cfg3_pin_fixture_rejects_logprob_errors_and_nan_retries():
     np.testing.assert_allclose(torch.stack(res['samples']).numpy(), d['samples_%d' % ci], rtol=1e-5, atol=1e-5)
 
 
-@pytest.mark.skipif(not reference_available(), reason='/root/reference only exists in the build container')
 def test_cfg4_oracle_equals_reference_live():
-    """BASELINE config 4 exactly (oracle/cfg4.py): hamiltorch.sample_split_model == the oracle, bit for bit."""
-    import torch.utils.data as tud
-    from oracle import cfg4
+    """BASELINE config 4 exactly (oracle/cfg4.py): hamiltorch.sample_split_model == the oracle, bit for bit, against
+    the reference's output stored by oracle/ref_pins.py."""
     torch.set_num_threads(1)
-    ref = import_reference()
-    model, X, y = cfg4.problem()
-    descs = cfg4.descriptors(model, X, y)
-    D = descs[0].dim
-    init = ref.util.flatten(model).detach().clone()
-    loader = tud.DataLoader(tud.TensorDataset(X, y), batch_size=cfg4.N_ROWS // cfg4.M, shuffle=False)
-    kw = dict(num_samples=4, num_steps_per_sample=cfg4.L, step_size=cfg4.EPS, inv_mass=torch.ones(D))
-    torch.manual_seed(5)
-    r = ref.sample_split_model(model, loader, params_init=init, num_splits=cfg4.M, model_loss='regression',
-                               tau_out=cfg4.TAU_OUT, integrator=ref.Integrator.SPLITTING, verbose=False, **kw)
-    torch.manual_seed(5)
-    next(iter(loader))                       # the DataLoader's base-seed draw (see oracle/gen_golden.py)
-    o = O.sample_hmc(descs, init, split_scheme=O.SPLIT_SYM, **kw)
-    assert torch.equal(torch.stack(r), torch.stack(o['samples']))
+    d = np.load(ref_pins.PINS)
+    assert torch.equal(torch.from_numpy(d['cfg4_samples']), torch.stack(ref_pins.oracle_cfg4()['samples']))
